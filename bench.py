@@ -11,9 +11,14 @@ A step = one pass of the fused chain over the whole [65536, 4096] CF32 batch = O
 b200_chain_exec_host: the same batch from pinned HOST memory, H2D + kernel + D2H inside the timed region.
 Prints ONE JSON line on rank 0.
 
+`--steps` sets the number of timed steps of the headline and of every workload (the e2e variants time
+min(--steps, --e2e-steps) host round trips, the wideband collective variants at most 5 steps). `--dump-outputs DIR`
+writes what the timed path computed in its last step as DIR/<name>.npy (float32; outputs above 32 MB as a fixed, seeded
+sample of rows, whose indices are written as DIR/<name>_rows.npy); the inputs are seeded, so two builds can be compared
+output for output.
+
 Besides the headline the same line carries (each measured after the headline's timed region, each guarded: a failure
 is recorded as {"error": ...} and never touches the headline):
-  sustained      the same step timed over 200 launches (the 20-step driver run is a 13 ms burst)
   e2e_variants   the e2e metric through the REFERENCE's own Flowgraph with provider b200 (shim/, full D2H and with the
                  lineplot + waterfall consumers = display-sized D2H), and from CI8 host samples
   workloads.fir       BASELINE configs[2]: 127-tap FIR + decimate-by-8, 2^26 CF32 samples
@@ -412,6 +417,30 @@ class Env:
         return plan
 
 
+DUMP_BYTES = 32 << 20         # per output array; larger outputs are written as a seeded sample of rows
+
+
+def dump_output(env, directory, name, tensor):
+    """Writes `tensor` (what a caller of the timed path receives) as float32 `directory/<name>.npy`; complex values as
+    trailing (re, im) pairs. Beyond DUMP_BYTES a fixed, seeded sample of rows (axis 0) is written, with its row indices
+    in `<name>_rows.npy` (float64)."""
+    import numpy as np
+    if not directory:
+        return
+    torch = env.torch
+    t = torch.view_as_real(tensor) if tensor.is_complex() else tensor
+    if env.world > 1:
+        name = f"{name}_rank{env.rank}"
+    os.makedirs(directory, exist_ok=True)
+    row_bytes = max(1, t[0].numel() * 4)
+    if t.numel() * 4 > DUMP_BYTES:
+        keep = min(t.shape[0], max(1, DUMP_BYTES // row_bytes))
+        rows = np.sort(np.random.default_rng(0).choice(t.shape[0], size=keep, replace=False))
+        np.save(os.path.join(directory, f"{name}_rows.npy"), rows.astype(np.float64))
+        t = t[torch.from_numpy(rows).to(t.device)]
+    np.save(os.path.join(directory, f"{name}.npy"), t.float().cpu().numpy())
+
+
 def guarded(fn, *a, **kw):
     try:
         return fn(*a, **kw)
@@ -514,7 +543,7 @@ def e2e_ci8(env, plan, rows, coeff, scale, offset, steps):
 
 # ---- BASELINE configs[2]: FIR ----------------------------------------------------------------------
 
-def bench_fir(env, steps, warmup, with_cpu=False):
+def bench_fir(env, steps, warmup, with_cpu=False, dump=None):
     """127-tap FIR + decimate-by-8 over 2^26 CF32 samples ([8192, 8192] frames, one stream): b200_fir_exec.
     Algorithmic bytes 8 + 8/R = 9 per input sample. L2: 512 MiB in + 64 MiB out per step >> 126 MB."""
     import numpy as np
@@ -534,6 +563,7 @@ def bench_fir(env, steps, warmup, with_cpu=False):
     def step():
         env.check(lib.b200_fir_exec(plan, x.data_ptr(), y.data_ptr(), frames, t, env.sp))
     ms, ms_max, t0, t1 = env.timed(step, steps, warmup)
+    dump_output(env, dump, "fir_out", y)
     samples = frames * t
     # e2e: pinned host frames -> device -> decimated result back, through the C ABI's own copies
     x_host = torch.empty(frames, t, dtype=torch.complex64, pin_memory=True)
@@ -627,7 +657,7 @@ def bench_fft(env, steps, warmup):
 
 # ---- BASELINE configs[3]: FM-broadcast flowgraph at 10 MS/s ---------------------------------------------
 
-def bench_fm(env, steps, warmup, with_cpu=False):
+def bench_fm(env, steps, warmup, with_cpu=False, dump=None):
     """Filter(161 taps, decimate 40) -> FM(narrow, 75 us) -> Filter(41 taps, decimate 2) -> Amplitude on one second of
     10 MS/s IQ ([2500, 4000] frames), module kernels back to back on one stream through the C ABI."""
     import numpy as np
@@ -668,6 +698,7 @@ def bench_fm(env, steps, warmup, with_cpu=False):
         env.check(lib.b200_fir_exec(p2, audio_c.data_ptr(), y2.data_ptr(), frames, t1, env.sp))
         env.check(lib.b200_amplitude_cf32(env.ctx.handle, y2.data_ptr(), db.data_ptr(), frames * t2, coeff, env.sp))
     ms, ms_max, _, _ = env.timed(step, steps, warmup)
+    dump_output(env, dump, "fm_out", db)
     for plan, destroy in ((p1, lib.b200_fir_plan_destroy), (p2, lib.b200_fir_plan_destroy), (pfm, lib.b200_fm_plan_destroy)):
         env.check(destroy(plan))
     value = samples * env.world / (ms_max * 1e-3) / 1e6
@@ -689,7 +720,7 @@ def bench_fm(env, steps, warmup, with_cpu=False):
 
 # ---- BASELINE configs[4]: 8-channel wideband chain, strong-scaled with the NCCL boundary collective ---------
 
-def bench_wideband(env, steps, warmup):
+def bench_wideband(env, steps, warmup, dump=None):
     """[8, 131072, 4096] CF32 = 2^20 rows, cut into `world` contiguous slabs (one channel per GPU at N = 8). Timed:
     (a) kernel only (every rank its slab, no collective); (b) kernel + gather of the FULL F32 result on rank 0 over NCCL
     (dist.gather, 2^20 x 4096 x 4 B = 16 GiB in total); (c) kernel with fused column sums + the DISPLAY-sized boundary:
@@ -729,6 +760,7 @@ def bench_wideband(env, steps, warmup):
     def kernel():
         env.check(lib.b200_chain_exec(plan, x.data_ptr(), out.data_ptr(), rows, coeff, 1, scale, offset, env.sp))
     ms_k, ms_k_max, _, _ = env.timed(kernel, steps, warmup)
+    dump_output(env, dump, "wideband_out", out)
 
     result = {"rows_total": WIDEBAND_ROWS, "rows_per_rank": rows, "scaling": "strong",
               "kernel_only": {"ms_per_step": ms_k_max, "value": WIDEBAND_ROWS * n / (ms_k_max * 1e-3) / 1e6, "unit": UNIT}}
@@ -797,18 +829,10 @@ def main_chain(env, args):
     sampler = ClockSampler(env.local)
     sampler.start()
     ms_local, ms_per_step, t_begin, t_end = env.timed(step, args.steps, args.warmup)
+    dump_output(env, args.dump_outputs, "chain_out", out)
     samples_per_step_all = rows * n * world
     value = samples_per_step_all / (ms_per_step * 1e-3) / 1e6
     launches = args.steps
-
-    # -- sustained: the same step over 200 launches (0.13 s) — the 20-step driver run is a 13 ms burst
-    sustained = None
-    if args.steps < 200 and not args.no_extras:
-        s_local, s_max, _, _ = env.timed(step, 200, 0)
-        ach = rows * n * BYTES_PER_SAMPLE / (s_local * 1e-3) / 1e9
-        sustained = {"steps": 200, "ms_per_step": s_max, "value": samples_per_step_all / (s_max * 1e-3) / 1e6,
-                     "unit": UNIT, "roofline_frac": ach / env.peak}
-        launches += 200
 
     # -- e2e: host buffers through b200_chain_exec_host (H2D + kernel + D2H every step)
     e2e_steps = max(1, min(args.steps, args.e2e_steps))
@@ -851,11 +875,11 @@ def main_chain(env, args):
     del x, out, x_host
     torch.cuda.empty_cache()
     if not args.no_extras:
-        workloads = {"wideband": guarded(bench_wideband, env, max(5, min(args.steps, 20)), 3)}
+        workloads = {"wideband": guarded(bench_wideband, env, args.steps, 3)}
         if world == 1:
-            workloads["fir"] = guarded(bench_fir, env, 50, 5)
-            workloads["fm"] = guarded(bench_fm, env, 50, 5)
-            workloads["fft"] = guarded(bench_fft, env, 20, 3)
+            workloads["fir"] = guarded(bench_fir, env, args.steps, 5)
+            workloads["fm"] = guarded(bench_fm, env, args.steps, 5)
+            workloads["fft"] = guarded(bench_fft, env, args.steps, 3)
         for w in workloads.values():
             if isinstance(w, dict):
                 launches += int(w.get("gpu_launches", 0) or 0)
@@ -881,7 +905,6 @@ def main_chain(env, args):
                     "api": "b200_chain_exec_host (pinned host buffers, 3-stream chunked pipeline)",
                     "checksum": checksum},
             "roofline": roofline,
-            "sustained": sustained,
             "cpu_baseline": cpu_baseline,
             "e2e_variants": variants,
             "workloads": workloads,
@@ -894,9 +917,9 @@ def main_chain(env, args):
 def main_single_workload(env, args):
     fn = {"fir": bench_fir, "fm": bench_fm}.get(args.workload)
     if fn is not None:
-        res = fn(env, args.steps, args.warmup, with_cpu=not args.no_cpu_baseline)
+        res = fn(env, args.steps, args.warmup, with_cpu=not args.no_cpu_baseline, dump=args.dump_outputs)
     else:
-        res = bench_wideband(env, args.steps, args.warmup)
+        res = bench_wideband(env, args.steps, args.warmup, dump=args.dump_outputs)
         res = {"metric": WORKLOAD_METRICS["wideband"], "value": res["kernel_only"]["value"], "unit": UNIT,
                "ms_per_step": res["kernel_only"]["ms_per_step"], "steps": args.steps,
                "config": {"workload": "wideband [8,131072,4096] CF32 strong-scaled", "l2": "inputs larger than L2"},
@@ -956,8 +979,14 @@ def main():
     ap.add_argument("--rows", type=int, default=ROWS)
     ap.add_argument("--e2e-steps", type=int, default=5)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--no-extras", action="store_true", help="headline only (no sustained / variants / workloads)")
+    ap.add_argument("--no-extras", action="store_true", help="headline only (no variants / workloads)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed path's outputs of its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's CUDA path; --impl reference has none")
     if args.impl == "reference":
         return main_reference(args)
     return main_ours(args)

@@ -12,10 +12,16 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu on the GPU box)")
 
 
-@pytest.fixture(scope="session")
-def ref():
-    """The reference CPU path (oracle/_ref/libjst_ref.so). Checker only."""
-    from oracle import ref as _ref
-    if not _ref.available():
-        pytest.skip("oracle/_ref/libjst_ref.so not built (needs /root/reference at build time)")
-    return _ref
+@pytest.fixture
+def ref(request):
+    """The reference CPU path (oracle/ref.py) for this test: its stored outputs, or the live library while recording
+    them (tests/reference_outputs.py). Checker only."""
+    from reference_outputs import Reference
+    node = request.node
+    return Reference(os.path.relpath(str(node.path), ROOT).replace(os.sep, "/") + "::" + node.name)
+
+
+def pytest_sessionfinish(session):
+    from reference_outputs import RECORD, STORE
+    if RECORD and STORE.recorded:
+        STORE.save()

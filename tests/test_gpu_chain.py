@@ -8,10 +8,9 @@ pytestmark = pytest.mark.gpu
 from parity import assert_db_close, true_spectrum
 
 
-def _window(ref, n):
-    w = ref.window(n).copy()
-    w[1::2] *= -1          # invert (even n): (-1)^k
-    return w
+def _window(n):
+    from oracle import port
+    return port.invert(port.window(n))          # the reference's taps, bit-exact (test_oracle), sign-flipped
 
 
 def _run_chain(x, enable_scale, rmin=-120.0, rmax=0.0, fused=True):
@@ -38,7 +37,7 @@ def test_chain_4096_scale(ref, rows):
     want = ref.spectrum_engine(x, enable_scale=True)
     got = _run_chain(x, True)
     assert got.shape == want.shape and got.dtype == np.float32
-    spec = true_spectrum(x, _window(ref, 4096))
+    spec = true_spectrum(x, _window(4096))
     assert_db_close(got, want, spec, scale=_range_slope(-120.0, 0.0), floor=3e-7)
 
 
@@ -47,7 +46,7 @@ def test_chain_4096_db(ref):
     x = spectral_rows(1000, 128)
     want = ref.spectrum_engine(x, enable_scale=False)
     got = _run_chain(x, False)
-    assert_db_close(got, want, true_spectrum(x, _window(ref, 4096)))
+    assert_db_close(got, want, true_spectrum(x, _window(4096)))
 
 
 def test_chain_4096_unfused_modules_match_fused(ref):
@@ -56,7 +55,7 @@ def test_chain_4096_unfused_modules_match_fused(ref):
     from cyberether_b200.synthetic import spectral_rows
     x = spectral_rows(50, 32)
     want = ref.spectrum_engine(x, enable_scale=True)
-    spec = true_spectrum(x, _window(ref, 4096))
+    spec = true_spectrum(x, _window(4096))
     for fused in (False, True):
         got = _run_chain(x, True, fused=fused)
         assert_db_close(got, want, spec, scale=_range_slope(-120.0, 0.0), floor=3e-7)
@@ -79,7 +78,7 @@ def test_chain_other_sizes(ref, n):
     x = spectral_rows(7, 5, n=n)
     want = ref.spectrum_engine(x, enable_scale=True, range_min=-100.0, range_max=-10.0)
     got = _run_chain(x, True, -100.0, -10.0)
-    assert_db_close(got, want, true_spectrum(x, _window(ref, n)), scale=_range_slope(-100.0, -10.0), floor=3e-7)
+    assert_db_close(got, want, true_spectrum(x, _window(n)), scale=_range_slope(-100.0, -10.0), floor=3e-7)
 
 
 @pytest.mark.parametrize("n", [16384, 65536])
@@ -89,21 +88,22 @@ def test_chain_tiled_two_pass_in_several_chunks_and_db_mode(ref, n, monkeypatch)
     from cyberether_b200.synthetic import spectral_rows
     monkeypatch.setenv("B200_FFT_TWOPASS_CHUNK_MB", str(max(1, (2 * n * 8) >> 20)))
     x = spectral_rows(11, 5, n=n)
-    spec = true_spectrum(x, _window(ref, n))
+    spec = true_spectrum(x, _window(n))
     assert_db_close(_run_chain(x, False), ref.spectrum_engine(x, enable_scale=False), spec)
     want = ref.spectrum_engine(x, enable_scale=True, range_min=-90.0, range_max=-20.0)
     assert_db_close(_run_chain(x, True, -90.0, -20.0), want, spec, scale=_range_slope(-90.0, -20.0), floor=3e-7)
     zero = np.zeros((3, n), np.complex64)
     assert np.all(np.isneginf(_run_chain(zero, False)))
-    assert np.array_equal(_run_chain(zero, True), ref.spectrum_engine(zero, enable_scale=True))
+    assert ref.spectrum_engine(zero, enable_scale=True).equals(_run_chain(zero, True))
 
 
 def test_chain_zero_input(ref):
     x = np.zeros((2, 4096), np.complex64)
-    assert np.array_equal(_run_chain(x, True), ref.spectrum_engine(x, enable_scale=True))
+    assert ref.spectrum_engine(x, enable_scale=True).equals(_run_chain(x, True))
     got = _run_chain(x, False)
     assert np.all(np.isneginf(got))
-    assert np.all(np.isneginf(ref.spectrum_engine(x, enable_scale=False)))
+    want = ref.spectrum_engine(x, enable_scale=False)
+    assert want.idx.size == want.size and np.all(np.isneginf(want.values))   # non-finite outputs are all stored
 
 
 def test_chain_flat_range(ref):
@@ -112,7 +112,7 @@ def test_chain_flat_range(ref):
     x = spectral_rows(3, 2)
     want = ref.spectrum_engine(x, enable_scale=True, range_min=-50.0, range_max=-50.0)
     got = _run_chain(x, True, -50.0, -50.0)
-    assert np.array_equal(got, want) and np.all(got == 0.5)
+    assert want.equals(got) and np.all(got == 0.5)
 
 
 def _chain_module(buffer, window, dtype=None, enable_scale=True, agc=False):
@@ -148,7 +148,7 @@ def test_chain_integer_ingest_equals_cast_then_chain(ref, name, np_type, n, rows
     mid = 0.0 if info.min < 0 else half
     x = np.stack([sig.real, sig.imag], axis=-1) * half * 0.9 + mid
     x = np.clip(np.rint(x), info.min, info.max).astype(np_type)
-    w = _window(ref, n)
+    w = _window(n)
     got = _chain_module(x, w, dtype=name, enable_scale=enable_scale)
     xf = port.cast(x, complex_pairs=True)                    # bit-exact restatement of the reference cast (test_oracle)
     two_step = _chain_module(xf, w, enable_scale=enable_scale)
@@ -192,7 +192,7 @@ def test_spectrum_engine_with_agc(ref, enable_scale, fused, n, level):
     want = ref.run_block("spectrum_engine", {"buffer": x}, {"enableAgc": True, "enableScale": enable_scale,
                                                            "rangeMin": -120.0, "rangeMax": 0.0}, "buffer")
     # the gain is common to a row: the allowance is computed on the spectrum the amplitude stage sees (g X)
-    w = _window(ref, n)
+    w = _window(n)
     spec = true_spectrum(x, w)
     mean_power = (np.abs(spec) ** 2).mean(axis=1, keepdims=True)
     gain = np.clip(1.0 / np.sqrt(mean_power + 1e-12), 0.01, 100.0)
@@ -203,12 +203,12 @@ def test_spectrum_engine_with_agc(ref, enable_scale, fused, n, level):
 
 
 @pytest.mark.parametrize("name,np_type", [("CI8", np.int8), ("CU16", np.uint16)])
-def test_chain_integer_ingest_with_agc(ref, name, np_type):
+def test_chain_integer_ingest_with_agc(name, np_type):
     """Integer ingest and the AGC stage in the same kernel: bit-identical to cast -> CF32 chain with AGC."""
     from oracle import port
     info = np.iinfo(np_type)
     x = np.random.default_rng(11).integers(info.min // 4, info.max // 4, size=(33, 4096, 2), dtype=np_type)
-    w = _window(ref, 4096)
+    w = _window(4096)
     got = _chain_module(x, w, dtype=name, agc=True)
     two_step = _chain_module(port.cast(x, complex_pairs=True), w, agc=True)
     assert np.array_equal(got, two_step)
@@ -237,7 +237,7 @@ def test_chain_full_size_rows_are_independent(ref):
              np.random.default_rng(5).integers(0, rows, 53)]
     small_in = torch.from_numpy(spectral_rows(0, 64)).to(dev)
     x[torch.tensor(picks[:8], device=dev)] = small_in[:8]              # a few rows the reference has seen
-    win = torch.from_numpy(_window(ref, n)).to(dev)
+    win = torch.from_numpy(_window(n)).to(dev)
     coeff = cb.amplitude_scaling_coeff(n)
     sc, off = cb.range_coefficients(-120.0, 0.0)
     stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
@@ -253,14 +253,19 @@ def test_chain_full_size_rows_are_independent(ref):
     assert torch.equal(big[torch.tensor(picks, device=dev)], sub)
     assert bool(torch.isfinite(big).all()) and float(big.min()) >= 0.0 and float(big.max()) <= 1.0
     want = ref.spectrum_engine(spectral_rows(0, 8), enable_scale=True)
-    spec = true_spectrum(spectral_rows(0, 8), _window(ref, n))
+    spec = true_spectrum(spectral_rows(0, 8), _window(n))
     assert_db_close(sub[:8].cpu().numpy(), want, spec, scale=_range_slope(-120.0, 0.0), floor=3e-7)
     # 1024 rows of the big launch against the reference CPU block (Gaussian rows: every bin is a "strong" bin)
     stride_rows = torch.arange(0, rows, 64, device=dev)
     x_host = x[stride_rows].cpu().numpy()
     want_many = ref.spectrum_engine(x_host, enable_scale=True)
     from parity import assert_strong_bins
-    spec_many = true_spectrum(x_host, _window(ref, n))
+    spec_many = true_spectrum(x_host, _window(n))
     got_many = big[stride_rows].cpu().numpy()
     assert_db_close(got_many, want_many, spec_many, scale=_range_slope(-120.0, 0.0), floor=3e-7)
     assert_strong_bins(got_many, want_many, spec_many, slope=_range_slope(-120.0, 0.0), label="full-size rows")
+    # every element of the 1024 rows: against the numpy restatement of the reference chain (another FP32 FFT)
+    from oracle import port
+    whole = port.spectrum_engine(x_host, enable_scale=True)
+    assert_db_close(got_many, whole, spec_many, scale=_range_slope(-120.0, 0.0), floor=3e-7)
+    assert_strong_bins(got_many, whole, spec_many, slope=_range_slope(-120.0, 0.0), label="full-size rows vs port")

@@ -26,12 +26,13 @@ def _run(module_type, inputs, config=None, out="signal", axes=None):
 def test_window_matches_reference(ref, n):
     got = _run("window", {}, {"size": n}, out="window")
     want = ref.window(n)
-    assert got.dtype == np.complex64 and got.shape == (n,)
+    assert got.dtype == np.complex64 and got.shape == want.shape == (n,)
     # F64 cos on the device vs glibc: identical after rounding to F32 except for rare double-rounding ties.
-    ulp = np.spacing(np.abs(want.real).astype(np.float32)).max()
-    assert np.abs(got.real - want.real).max() <= ulp
+    g, w = want.take(got), want.values
+    ulp = np.spacing(np.abs(w.real).astype(np.float32)).max()
+    assert np.abs(g.real - w.real).max() <= ulp
     assert np.all(got.imag == 0)
-    assert float((got.real != want.real).mean()) < 1e-3
+    assert float((g.real != w.real).mean()) < 1e-3
 
 
 def test_window_formula_known_answer():
@@ -50,9 +51,11 @@ def test_invert_bit_exact(ref, shape, axis):
     got = _run("invert", {"signal": x})
     want = ref.run_block("invert", {"signal": x}, None, "signal")
     if shape[axis] % 2 == 0:
-        assert np.array_equal(got, want)          # sign flips are exact
+        assert want.equals(got)                   # sign flips are exact
+        from oracle import port                   # the whole output: the restatement pinned to the reference
+        assert np.array_equal(got, port.invert(x, axis))
     else:
-        assert np.abs(got - want).max() <= 2 * np.spacing(np.float32(np.abs(want).max()))
+        assert np.abs(want.diff(got)).max() <= 2 * np.spacing(np.float32(want.absmax()))
 
 
 @pytest.mark.parametrize("sa,sb", [((64, 4096), (1, 4096)), ((64, 4096), (64, 4096)), ((4, 3, 8), (3, 1)),
@@ -66,17 +69,18 @@ def test_multiply_cf32_bit_exact(ref, sa, sb):
     want = ref.run_block("multiply", {"a": a, "b": b}, None, "product",
                          axes={"a": (len(sa) - 1, -1, -1), "b": (len(sb) - 1, -1, -1)})
     assert got.shape == want.shape
-    assert np.array_equal(got, want)
+    assert want.equals(got)
+    from oracle import port                       # the whole output: the restatement pinned to the reference
+    assert np.array_equal(got, port.multiply(a, b))
 
 
 def test_multiply_conflicting_axes_rejected_like_reference(ref):
     """Batch roles that right-align to different output axes are an ERROR in the reference
     ("Signal roles map to conflicting output axes"); the mirror rejects the same graph."""
     import cyberether_b200 as cb
-    from oracle.ref import RefError
     from cyberether_b200.synthetic import gaussian_cf32
     a, b = gaussian_cf32((4, 3, 8), 1), gaussian_cf32((3, 1), 2)
-    with pytest.raises(RefError):
+    with pytest.raises(ref.RefError):
         ref.run_block("multiply", {"a": a, "b": b}, None, "product", axes={"a": (2, 0, -1), "b": (1, 0, -1)})
     ctx = cb.TestContext("multiply")
     ctx.set_input("a", a, sampleAxis=2, batchAxis=0)
@@ -89,7 +93,9 @@ def test_multiply_f32_bit_exact(ref):
     rng = np.random.default_rng(3)
     a = rng.standard_normal((128, 512)).astype(np.float32)
     b = rng.standard_normal((512,)).astype(np.float32)
-    assert np.array_equal(_run("multiply", {"a": a, "b": b}, out="product"), ref.multiply(a, b))
+    from oracle import port
+    got = _run("multiply", {"a": a, "b": b}, out="product")
+    assert ref.multiply(a, b).equals(got) and np.array_equal(got, port.multiply(a, b))
 
 
 @pytest.mark.parametrize("n", [2, 4, 8, 16, 32, 64, 128, 256, 512, 1024, 2048, 4096, 8192, 16384])
@@ -101,11 +107,11 @@ def test_fft_c2c_matches_reference(ref, n, forward):
     x = gaussian_cf32((rows, n), 100 + n)
     got = _run("fft", {"signal": x}, {"forward": forward})
     want = ref.fft(x, forward=forward)
-    rel = np.abs(got - want).max(axis=-1) / np.abs(want).max(axis=-1)
+    rel = np.abs(want.diff(got)) / want.row_absmax_at()
     assert rel.max() <= 2e-6, rel.max()
     exact = np.fft.fft(x.astype(np.complex128), axis=-1) if forward else np.fft.ifft(x.astype(np.complex128), axis=-1) * n
-    ours = np.abs(got - exact).max() / np.abs(exact).max()
-    theirs = np.abs(want - exact).max() / np.abs(exact).max()
+    ours = np.abs(want.diff(got) - (want.take(exact) - want.values)).max() / np.abs(exact).max()
+    theirs = np.abs(want.values - want.take(exact)).max() / np.abs(exact).max()
     assert ours <= 3 * theirs + 1e-7, (ours, theirs)    # no less accurate than pocketfft
 
 
@@ -136,7 +142,9 @@ def test_amplitude_cf32_bit_exact(ref):
     x[1, :4] = [1e-30, 1e30, 1 + 0j, 2 + 0j]
     got = _run("amplitude", {"signal": x})
     want = ref.amplitude(x)
-    assert np.array_equal(got, want)              # same operation order, no FMA: bit-identical
+    assert want.equals(got)                       # same operation order, no FMA: bit-identical
+    from oracle import port
+    assert np.array_equal(got, port.amplitude(x, 4096))
     assert np.all(np.isneginf(got[0, :8]))
 
 
@@ -144,7 +152,9 @@ def test_amplitude_f32_bit_exact(ref):
     rng = np.random.default_rng(4)
     x = (rng.standard_normal((16, 1000)) * 10).astype(np.float32)
     x[0, 0] = 0.0
-    assert np.array_equal(_run("amplitude", {"signal": x}), ref.amplitude(x))
+    from oracle import port
+    got = _run("amplitude", {"signal": x})
+    assert ref.amplitude(x).equals(got) and np.array_equal(got, port.amplitude(x, 1000))
 
 
 @pytest.mark.parametrize("lo,hi", [(-1.0, 1.0), (-120.0, 0.0), (0.0, -120.0), (5.0, 5.0)])
@@ -155,8 +165,8 @@ def test_range_matches_reference(ref, lo, hi):
     got = _run("range", {"signal": x}, {"min": lo, "max": hi})
     want = ref.range_(x, lo, hi)
     # CUDA tanhf vs glibc tanhf: <= 2 ulp of tanh -> <= 1.2e-7 absolute on [0, 1] (reference test: 1e-6).
-    assert np.abs(got - want).max() <= 2.5e-7
-    assert got[0, 0] == want[0, 0] and got[0, 1] == want[0, 1]
+    assert np.abs(want.diff(got)).max() <= 2.5e-7
+    assert np.array_equal(got.reshape(-1)[want.idx[:2]], want.values[:2]) and want.idx[1] == 1     # -inf and inf
 
 
 def test_cast_bypass_and_f32():
@@ -193,7 +203,7 @@ def test_fft_trailing_batch_axis(ref):
     want = ref.run_block("fft", {"signal": x}, {"forward": True}, "signal", axes={"signal": (0, 1, -1)})
     got = _run_view("fft", x, lambda t: t, {"sampleAxis": 0, "batchAxis": 1}, {"forward": True})
     assert got.shape == want.shape
-    assert np.abs(got - want).max() <= 2e-6 * np.abs(want).max()
+    assert np.abs(want.diff(got)).max() <= 2e-6 * want.absmax()
 
 
 def test_fft_rank3_heads_middle_sample_axis(ref):
@@ -201,7 +211,7 @@ def test_fft_rank3_heads_middle_sample_axis(ref):
     x = gaussian_cf32((3, 128, 5), 22)
     want = ref.run_block("fft", {"signal": x}, {"forward": False}, "signal", axes={"signal": (1, 0, 2)})
     got = _run_view("fft", x, lambda t: t, {"sampleAxis": 1, "batchAxis": 0, "channelAxis": 2}, {"forward": False})
-    assert np.abs(got - want).max() <= 2e-6 * np.abs(want).max()
+    assert np.abs(want.diff(got)).max() <= 2e-6 * want.absmax()
 
 
 def test_fft_strided_slice_view():
@@ -220,11 +230,11 @@ def test_amplitude_and_range_non_contiguous_bit_exact(ref):
     view = np.ascontiguousarray(base.transpose(1, 0, 2)[:, ::2, :])          # dense copy of what the view holds
     got = _run_view("amplitude", base, lambda t: t.permute(1, 0, 2)[:, ::2, :], {"sampleAxis": 2})
     want = ref.run_block("amplitude", {"signal": view}, None, "signal", axes={"signal": (2, -1, -1)})
-    assert np.array_equal(got, want)
+    assert want.equals(got)
     fbase = np.random.default_rng(1).standard_normal((6, 40)).astype(np.float32)
     got = _run_view("range", fbase, lambda t: t[:, ::4], {}, {"min": -2.0, "max": 2.0})
     want = ref.range_(np.ascontiguousarray(fbase[:, ::4]), -2.0, 2.0)
-    assert np.abs(got - want).max() <= 2.5e-7
+    assert np.abs(want.diff(got)).max() <= 2.5e-7
 
 
 # ---- real-input transforms ("FFT - Complex Real Signal F32", "FFT - FFTPACK Real ...", fft/module_tests.cc:149-440) ----
@@ -238,20 +248,22 @@ def test_fft_r2c_complex_output(ref, shape, axes):
     got = _run_view("fft", x, lambda t: t, {k: v for k, v in names.items() if v is not None},
                     {"forward": True, "complexOutput": True})
     assert got.shape == want.shape and got.dtype == np.complex64
-    assert np.abs(got - want).max() <= 2e-6 * np.abs(want).max()
+    assert np.abs(want.diff(got)).max() <= 2e-6 * want.absmax()
 
 
 @pytest.mark.parametrize("n", [8, 64, 2048])
 def test_fft_fftpack_real_forward_inverse(ref, n):
     rng = np.random.default_rng(32)
     x = rng.standard_normal((4, n)).astype(np.float32)
+    half_complex = rng.standard_normal((4, n)).astype(np.float32)        # any real row is an FFTPACK spectrum
     fwd_want = ref.run_block("fft", {"signal": x}, {"forward": True}, "signal")
+    inv_want = ref.run_block("fft", {"signal": half_complex}, {"forward": False}, "signal")
     fwd = _run("fft", {"signal": x}, {"forward": True})
     assert fwd.dtype == np.float32 and fwd.shape == (4, n)
-    assert np.abs(fwd - fwd_want).max() <= 2e-6 * np.abs(fwd_want).max()
-    inv_want = ref.run_block("fft", {"signal": fwd_want}, {"forward": False}, "signal")
-    inv = _run("fft", {"signal": fwd_want}, {"forward": False})
-    assert np.abs(inv - inv_want).max() <= 2e-6 * np.abs(inv_want).max()
+    assert np.abs(fwd_want.diff(fwd)).max() <= 2e-6 * fwd_want.absmax()
+    inv = _run("fft", {"signal": half_complex}, {"forward": False})
+    assert np.abs(inv_want.diff(inv)).max() <= 2e-6 * inv_want.absmax()
+    inv = _run("fft", {"signal": fwd}, {"forward": False})
     assert np.abs(inv / n - x).max() <= 1e-5          # unnormalised round trip (reference tolerance 1e-2)
 
 
@@ -262,7 +274,7 @@ def test_fft_large_power_of_two_four_step(ref, n):
     for forward in (True, False):
         got = _run("fft", {"signal": x}, {"forward": forward})
         want = ref.fft(x, forward=forward)
-        assert np.abs(got - want).max() <= 3e-6 * np.abs(want).max()
+        assert np.abs(want.diff(got)).max() <= 3e-6 * want.absmax()
 
 
 @pytest.mark.parametrize("n", [3, 5, 7, 12, 100, 1000, 4095, 4099, 8320])
@@ -273,7 +285,7 @@ def test_fft_arbitrary_length_bluestein(ref, n):
     for forward in (True, False):
         got = _run("fft", {"signal": x}, {"forward": forward})
         want = ref.fft(x, forward=forward)
-        assert np.abs(got - want).max() <= 1e-5 * np.abs(want).max()     # north-star tolerance
+        assert np.abs(want.diff(got)).max() <= 1e-5 * want.absmax()     # north-star tolerance
 
 
 def test_chain_non_power_of_two_length(ref):
@@ -291,8 +303,8 @@ def test_chain_non_power_of_two_length(ref):
     assert block.compute() == cb.Result.SUCCESS, cb.last_error()
     got = block.output("buffer").numpy()
     block.destroy()
-    w = ref.window(n).copy()
-    w[1::2] *= -1
+    from oracle import port
+    w = port.invert(port.window(n))
     assert_db_close(got, want, true_spectrum(x, w), scale=2.0 / 120.0, floor=3e-7)
 
 
@@ -306,22 +318,25 @@ CAST_CASES = [("I8", np.int8, False), ("U8", np.uint8, False), ("I16", np.int16,
 def test_cast_integer_bit_exact(ref, name, np_type, is_complex, shape):
     """cast: every integer / complex-integer conversion of the reference's native module, bit-exact, including the
     extreme values and sizes that exercise the vector body and the scalar tail."""
+    import zlib
     import cyberether_b200 as cb
     info = np.iinfo(np_type)
-    rng = np.random.default_rng(hash(name) % 1000)
+    rng = np.random.default_rng(zlib.crc32(name.encode()) % 1000)       # the same input in every process
     full = shape + (2,) if is_complex else shape
     x = rng.integers(info.min, info.max, size=full, endpoint=True, dtype=np_type)
     x.flat[0] = info.min
     x.flat[-1] = info.max
     out_type = "CF32" if is_complex else "F32"
+    want = ref.run_block("cast", {"buffer": x}, {"outputType": out_type}, "buffer", dtypes={"buffer": name})
     ctx = cb.TestContext("cast")
     ctx.set_input("buffer", x, dtype=name, sampleAxis=len(shape) - 1)
     ctx.set_config(outputType=out_type)
     assert ctx.run() == cb.Result.SUCCESS, cb.last_error()
     got = ctx.output("buffer")
-    want = ref.run_block("cast", {"buffer": x}, {"outputType": out_type}, "buffer", dtypes={"buffer": name})
     assert got.dtype == want.dtype and got.shape == want.shape == shape
-    assert np.array_equal(got, want)
+    assert want.equals(got)
+    from oracle import port                       # the whole output: the restatement pinned to the reference
+    assert np.array_equal(got, port.cast(x, complex_pairs=is_complex))
 
 
 def test_cast_unsupported_pair_is_an_error():
@@ -337,6 +352,8 @@ def _assert_agc_equal(got, want):
     """Gains are F64 on both sides and differ only by the order of the F64 power sum (a few F64 ulp), so the F32
     outputs are identical except for rare last-bit rounding flips."""
     assert got.shape == want.shape and got.dtype == want.dtype
+    if hasattr(want, "row_absmax"):                 # a stored sample of the reference output
+        got, want = want.take(got), want.values
     g = got.view(np.float32) if np.iscomplexobj(got) else got
     w = want.view(np.float32) if np.iscomplexobj(want) else want
     both_nan = np.isnan(g) & np.isnan(w)

@@ -31,7 +31,7 @@ def _ref_lineplot(ref, cycles, config, axes):
     with ref.VizSession("lineplot", cycles[0].shape, config, **kw) as v:
         for x in cycles:
             v.compute(x)
-            outs.append(v.read().reshape(-1, 2))
+            outs.append(v.read(select=lambda a: a.reshape(-1, 2)))
     return outs
 
 
@@ -51,7 +51,14 @@ def test_lineplot_small_batches_bit_exact(ref, shape, config, axes):
     got = _lineplot(cycles, config, axes)
     want = _ref_lineplot(ref, cycles, config, axes)
     for g, w in zip(got, want):
-        assert np.array_equal(g, w)
+        assert w.equals(g)
+    if axes == {"sampleAxis": 1, "batchAxis": 0}:
+        # the whole output: the restatement pinned to the reference (batch-leading layout)
+        from oracle import port
+        p = port.Lineplot(shape[1], batches=shape[0], decimation=config.get("decimation", 1),
+                          averaging=config.get("averaging", 1))
+        for g, x in zip(got, cycles):
+            assert np.array_equal(g, p.compute(x))
 
 
 def test_lineplot_nonfinite_input_is_clamped(ref):
@@ -60,7 +67,7 @@ def test_lineplot_nonfinite_input_is_clamped(ref):
     got = _lineplot(cycles, {"averaging": 2}, {"sampleAxis": 1, "batchAxis": 0})
     want = _ref_lineplot(ref, cycles, {"averaging": 2}, {"sampleAxis": 1, "batchAxis": 0})
     for g, w in zip(got, want):
-        assert np.all(np.isfinite(g)) and np.array_equal(g, w)
+        assert np.all(np.isfinite(g)) and np.array_equal(g, w.array())
 
 
 @pytest.mark.parametrize("shape,config", [((1000, 4096), {}), ((4096, 1024), {"decimation": 2, "averaging": 5}),
@@ -78,8 +85,9 @@ def test_lineplot_large_batches_within_reassociation_tolerance(ref, shape, confi
     want = _ref_lineplot(ref, cycles, config, axes)
     for g, a, w in zip(got, again, want):
         assert np.array_equal(g, a)
-        assert np.array_equal(g[:, 0], w[:, 0])
-        assert np.abs(g[:, 1] - w[:, 1]).max() <= 2e-6
+        column = w.idx % 2
+        assert np.array_equal(w.take(g)[column == 0], w.values[column == 0])
+        assert np.abs(w.diff(g)[column == 1]).max() <= 2e-6
 
 
 @pytest.mark.parametrize("batches,height,n", [(1, 5, 3), (5, 5, 3), (6, 5, 3), (13, 5, 8), (3, 5, 8), (700, 512, 4096),
@@ -88,6 +96,8 @@ def test_waterfall_ring_matches_reference(ref, batches, height, n):
     import cyberether_b200 as cb
     from cyberether_b200.blocks import WaterfallBlock
     import torch
+    from oracle import port
+    expected = port.Waterfall(n, height)              # the whole ring: the restatement pinned to the reference
     rng = np.random.default_rng(2)
     cycles = [rng.standard_normal((batches, n)).astype(np.float32) for _ in range(4)]
     inp = cb.Tensor.from_numpy(cycles[0], sampleAxis=1, batchAxis=0)
@@ -98,8 +108,9 @@ def test_waterfall_ring_matches_reference(ref, batches, height, n):
             inp.data.copy_(torch.from_numpy(x))
             assert block.compute() == cb.Result.SUCCESS, cb.last_error()
             v.compute(x)
-            assert np.array_equal(block.frequency_bins(), v.read().reshape(height, n))
+            assert v.read(select=lambda a: a.reshape(height, n)).equals(block.frequency_bins())
             assert block.write_index == v.write_index()
+            assert np.array_equal(block.frequency_bins(), expected.compute(x)) and block.write_index == expected.write_index
     block.destroy()
 
 
@@ -175,11 +186,11 @@ def test_fused_chain_column_sums_feed_the_lineplot(ref, rows, scale, dtype):
         # (b) the reference chain + reference lineplot on the CPU (CF32 only; the reference has no fused integer ingest)
         if dtype == "CF32":
             want_spectra = ref.spectrum_engine(x, enable_scale=scale)
-            ref_lp.compute(np.where(np.isfinite(want_spectra), want_spectra, want_spectra))
-            w = ref_lp.read().reshape(-1, 2)
+            ref_lp.compute(want_spectra)
+            w = ref_lp.read(select=lambda a: a.reshape(-1, 2))
             # spectra differ within the chain allowance (noise-floor bins up to ~0.2 dB); averaged over `rows` and
             # mapped to [-1, 1]: dB outputs are clamped at -1 (all far below 0), range outputs compared at 2e-4
-            assert np.abs(g[:, 1] - w[:, 1]).max() <= (2e-4 if scale else 1e-6)
+            assert np.abs(w.diff(g)[w.idx % 2 == 1]).max() <= (2e-4 if scale else 1e-6)
     ref_lp.close()
     fused.destroy()
     plain.destroy()

@@ -88,14 +88,17 @@ def test_cast_bypass_aliases_input():
 
 
 def test_spectrum_engine_wiring_fused_and_unfused():
-    x = tensor((64, 4096), sampleAxis=1, batchAxis=0)
+    import torch
+    # the input lives where the block's input-less modules (window) allocate: the CUDA device when one is visible
+    x = cb.Tensor.from_numpy(np.zeros((64, 4096), np.complex64), device="cuda" if torch.cuda.is_available() else "cpu",
+                             sampleAxis=1, batchAxis=0)
     fused = SpectrumEngine(enableScale=True)
-    assert fused.create("spec", {"buffer": x}) == cb.Result.SUCCESS
+    assert fused.create("spec", {"buffer": x}) == cb.Result.SUCCESS, cb.last_error()
     assert list(fused.modules) == ["cast_input", "window", "invert", "spectral_chain"]
     out = fused.output("buffer")
     assert out.shape == (64, 4096) and out.dtype == "F32" and out.attribute("sampleAxis") == 1
     unfused = SpectrumEngine(enableScale=True, fused=False)
-    assert unfused.create("spec", {"buffer": x}) == cb.Result.SUCCESS
+    assert unfused.create("spec", {"buffer": x}) == cb.Result.SUCCESS, cb.last_error()
     assert list(unfused.modules) == ["cast_input", "window", "invert", "reshape_window", "multiply", "fft",
                                      "amplitude", "range"]       # the reference's own sequence (block_impl.cc:120-217)
     order = [m.name.split(":")[1] for m in unfused.scheduler.order]
@@ -105,12 +108,12 @@ def test_spectrum_engine_wiring_fused_and_unfused():
     static = {m.name.split(":")[1] for m in sched.order if sched.is_static(m)}
     assert static == {"window", "invert", "reshape_window"}     # settle after cycle 1 (block_tests.cc:103-122)
     with_agc = SpectrumEngine(enableAgc=True, fused=False)      # agc sits between fft and amplitude (block_impl.cc:186-200)
-    assert with_agc.create("s", {"buffer": x}) == cb.Result.SUCCESS
+    assert with_agc.create("s", {"buffer": x}) == cb.Result.SUCCESS, cb.last_error()
     names = list(with_agc.modules)
     assert names.index("fft") < names.index("agc") < names.index("amplitude") and "spectral_chain" not in names
     assert with_agc.modules["agc"].config["tileSize"] == 4096   # one RMS tile per spectrum
     fused_agc = SpectrumEngine(enableAgc=True)                  # 4096-point spectra: the stage lives inside the fused kernel
-    assert fused_agc.create("s", {"buffer": x}) == cb.Result.SUCCESS
+    assert fused_agc.create("s", {"buffer": x}) == cb.Result.SUCCESS, cb.last_error()
     assert "agc" not in fused_agc.modules and fused_agc.modules["spectral_chain"].config["enableAgc"] is True
     assert SpectrumEngine().create("s", {"buffer": tensor((4, 8))}) == cb.Result.ERROR
 
